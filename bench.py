@@ -115,6 +115,47 @@ class ClockSampler:
                 "samples": len(sm), "window": window}
 
 
+DUMP_BYTES = 63 << 20  # array data of --dump-outputs; the rest of 64 MB is left for the .npy headers
+
+
+def download_block(L, dev, blk):
+    """Host copies (numpy) of the columns of a library-owned DEVICE result block; NULLs become NaN."""
+    import numpy as np
+    from databend_b200 import lib
+    from databend_b200.block import np_dtype
+    cols = []
+    for i in range(blk.num_cols):
+        c = blk.cols[i]
+        a = np.empty(c.len, dtype=np_dtype(c.dtype))
+        if c.len:
+            lib.check(L.dbx_memcpy_d2h(dev, a.ctypes.data, c.data, a.nbytes))
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if c.validity and c.len:
+            vb = np.empty((c.validity_bit_offset + c.len + 7) // 8, dtype=np.uint8)
+            lib.check(L.dbx_memcpy_d2h(dev, vb.ctypes.data, c.validity, vb.nbytes))
+            valid = np.unpackbits(vb, bitorder="little")[c.validity_bit_offset:c.validity_bit_offset + c.len]
+            a[valid == 0] = np.nan
+        cols.append(a)
+    return cols
+
+
+def write_outputs(out_dir, tables):
+    """--dump-outputs: `tables` maps a table to {name: array}; the arrays of one table share their
+    first dimension.  Written as <out_dir>/<name>.npy in float32/float64.  When everything together
+    exceeds DUMP_BYTES, every table keeps the same fraction of its rows, chosen by a fixed seed, so
+    two builds run with the same arguments write the same rows."""
+    import numpy as np
+    total = sum(a.nbytes for t in tables.values() for a in t.values())
+    frac = min(1.0, DUMP_BYTES / total) if total else 1.0
+    os.makedirs(out_dir, exist_ok=True)
+    for cols in tables.values():
+        n = len(next(iter(cols.values())))
+        m = int(n * frac)
+        keep = np.sort(np.random.default_rng(0).choice(n, m, replace=False)) if m < n else slice(None)
+        for name, a in cols.items():
+            np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[keep]))
+
+
 def make_query():
     from databend_b200 import expr as E
     from databend_b200.transforms import AggregatorParams
@@ -178,7 +219,8 @@ def run_reference(args):
 # ---------------------------------------------------------------------------------- kNN leg
 def run_knn(args, L, dev, rank, world, barrier):
     """configs[4]: cosine_distance brute-force kNN, corpus sharded by rows across ranks, queries
-    replicated; per-rank top-k all-gathered and merged.  Returns the "knn" object of the JSON line."""
+    replicated; per-rank top-k all-gathered and merged.  Returns the "knn" object of the JSON line
+    and the (row ids, distances) of the last timed batch; (None, None) on ranks other than 0."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -242,7 +284,7 @@ def run_knn(args, L, dev, rank, world, barrier):
     stats = op.stats()
     op.close()
     if rank != 0:
-        return None
+        return None, None
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     peak, src = 1400.0, "fallback (B200_PROFILING.md sustained)"
     if os.path.exists(p):
@@ -280,7 +322,7 @@ def run_knn(args, L, dev, rank, world, barrier):
         dt = time.perf_counter() - t0
         out["cpu_baseline"] = {"value": sq / dt * sn / n_total, "unit": "queries/s", "cores": threads, "kind": "port",
                                "sample": f"{sq} queries x {sn} rows, row-wise cosine_distance (oracle, OpenMP) + top-k, scaled by {sn}/{n_total} rows"}
-    return out
+    return out, res
 
 # ---------------------------------------------------------------------------------- GPU arm
 def verify_result(out_block, dev, rank, world, cols, n, keys_total, torch, dist):
@@ -502,13 +544,14 @@ def run_dbx(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def run_steps(blocks, steps, out_mem, timed):
+    def run_steps(blocks, steps, out_mem, timed, keep_last=False):
+        """keep_last: return the last step's device result block itself (the caller releases it)."""
         res = None
         for i in range(steps):
             res = step_device(blocks, out_mem, prefetch_next=(i + 1 < steps))
             if timed:
                 step_walls.append(time.perf_counter())
-            if out_mem == abi.MEM_DEVICE:
+            if out_mem == abi.MEM_DEVICE and not (keep_last and i + 1 == steps):
                 rows_out = res.num_rows
                 L.dbx_block_release(C.byref(res))
                 res = rows_out
@@ -528,12 +571,22 @@ def run_dbx(args):
     ev1 = torch.cuda.Event(enable_timing=True)
     ev0.record(part_stream)
     t0 = time.perf_counter()
-    groups = run_steps([dblock], args.steps, abi.MEM_DEVICE, True)
+    groups = run_steps([dblock], args.steps, abi.MEM_DEVICE, True, keep_last=bool(args.dump_outputs))
     ev1.record(fin_stream)
     barrier()
     wall = time.perf_counter() - t0
     sampler.mark()
     gc.enable()
+    agg_out = None
+    if args.dump_outputs:  # the last timed step's result, as the caller of the operator receives it
+        last = groups
+        groups = last.num_rows
+        agg_out = download_block(L, dev, last)
+        L.dbx_block_release(C.byref(last))
+        if world > 1:  # every rank owns a disjoint set of groups
+            parts = [None] * world
+            dist.all_gather_object(parts, agg_out)
+            agg_out = [np.concatenate(c) for c in zip(*parts)]
     dev_ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if rank == 0 else None
     launches = L.dbx_kernel_launch_count() - launches0
@@ -620,8 +673,9 @@ def run_dbx(args):
     fin.close()
     for b_ in bufs:
         b_.free()
+    knn_out = None
     if not args.no_knn:
-        knn = run_knn(args, L, dev, rank, world, barrier)
+        knn, knn_out = run_knn(args, L, dev, rank, world, barrier)
 
     if rank != 0:
         if world > 1:
@@ -673,6 +727,13 @@ def run_dbx(args):
         "cpu_baseline": cpu, "e2e": e2e, "knn": knn,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        # group order out of the hash table is unspecified: rows are written in ascending key order
+        o = np.argsort(agg_out[3], kind="stable")
+        tables = {"agg": {name: agg_out[i][o] for i, name in enumerate(["agg_sum_v", "agg_count_v", "agg_avg_x", "agg_k"])}}
+        if knn_out is not None:
+            tables["knn"] = {"knn_row_id": knn_out[0].astype(np.float64), "knn_distance": knn_out[1].astype(np.float32)}
+        write_outputs(args.dump_outputs, tables)
     if world > 1:
         dist.destroy_process_group()
 
@@ -698,7 +759,16 @@ def main():
     ap.add_argument("--knn-queries", type=int, default=1024)
     ap.add_argument("--knn-k", type=int, default=10)
     ap.add_argument("--knn-cpu-rows", type=int, default=1_000_000, help="corpus rows of the CPU sample in the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32/float64, "
+                         "at most 64 MB in all: a fixed, seeded sample of the rows when larger): the query result in "
+                         "ascending key order (agg_sum_v, agg_count_v, agg_avg_x, agg_k; integers converted to float64) "
+                         "and the kNN leg's top-k per query (knn_row_id, knn_distance)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "dbx":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl dbx")
     if args.impl == "reference":
         run_reference(args)
     else:
