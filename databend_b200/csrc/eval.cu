@@ -240,18 +240,24 @@ extern "C" int32_t dbx_eval_scalar(int32_t device, const dbx_expr* expr, const d
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((n + 255) / 256, (int64_t)kNumSMs * 8));
     // A straight-line kernel generated for this expression (NVRTC, cached per expression shape, types
     // and literals); without NVRTC, or with DBX_EVAL_JIT=0, the interpreter serves it — same results.
+    // DBX_EVAL_JIT=2 is strict: a generated kernel that cannot be compiled or launched is an error
+    // instead of a silent fall-back, so a caller can prove the generated kernel ran.
     cudaKernel_t jk = nullptr;
     const char* jit_env = getenv("DBX_EVAL_JIT");
-    const bool jit_off = jit_env && atoi(jit_env) == 0;
-    if (!jit_off) {
-      std::string why;
-      if (!jit_get_kernel(specialised_source(p), "dbx_jit_eval", &jk, &why)) jk = nullptr;
-    }
+    const int jit_mode = jit_env ? atoi(jit_env) : 1;
+    std::string why;
+    if (jit_mode != 0 && !jit_get_kernel(specialised_source(p), "dbx_jit_eval", &jk, &why)) jk = nullptr;
     bool launched = false;
     if (jk) {
       void* args[] = {(void*)&p};
       const cudaError_t ce = cudaLaunchKernel((const void*)jk, dim3(grid), dim3(256), args, 0, st);
-      if (ce == cudaSuccess) launched = true; else cudaGetLastError();
+      if (ce == cudaSuccess) launched = true;
+      else { why = std::string("cudaLaunchKernel: ") + cudaGetErrorString(ce); cudaGetLastError(); }
+    }
+    if (!launched && jit_mode == 2) {
+      cudaStreamSynchronize(st);  // the input uploads still read host memory the caller may free
+      err.set("eval: DBX_EVAL_JIT=2 and the generated kernel did not run: " + why);
+      return DBX_ERR_UNSUPPORTED;
     }
     if (!launched) eval_kernel<<<grid, 256, 0, st>>>(p);
     count_launch();

@@ -84,6 +84,10 @@ __device__ __forceinline__ uint64_t f64_as_int(double d, int t) {
 // Rust `x as T` between any two numeric types (lossy where Rust is)
 __device__ __forceinline__ uint64_t cast_as(uint64_t v, int from, int to) {
   if (is_float_t(to)) {
+    // 64-bit integers round once, straight to f32 (cvt.rn.f32.{s64,u64}): through f64 they would round
+    // twice (2^60 + 2^36 + 1 -> 2^60 instead of 2^60 + 2^37).  Narrower integers are exact in f64.
+    if (to == DBX_F32 && from == DBX_I64) return (uint64_t)__double_as_longlong((double)__ll2float_rn((long long)v));
+    if (to == DBX_F32 && from == DBX_U64) return (uint64_t)__double_as_longlong((double)__ull2float_rn((unsigned long long)v));
     double d = as_f64(v, from);
     if (to == DBX_F32) d = (double)(float)d;
     return (uint64_t)__double_as_longlong(d);

@@ -471,7 +471,11 @@ int32_t dbx_op_kernel_variant(dbx_op* op, char* out, int32_t cap);
  * DBX_OK, or DBX_ERR_UNSUPPORTED with the reason in msg. */
 int32_t dbx_agg_jit_selftest(char* msg, int32_t msg_cap);
 /* Same for the scalar-expression evaluator: generates and compiles the straight-line kernel of a canned
- * expression (dbx_eval_scalar compiles one per expression shape; DBX_EVAL_JIT=0 keeps the interpreter). */
+ * expression (dbx_eval_scalar compiles one per expression shape; DBX_EVAL_JIT=0 keeps the interpreter).
+ * DBX_EVAL_JIT=2 is the strict form of the default: when the generated kernel cannot be compiled or
+ * launched, dbx_eval_scalar returns DBX_ERR_UNSUPPORTED with the reason (NVRTC's log) in the message
+ * instead of falling back to the interpreter.  Unset or any other non-zero value: generated kernel,
+ * interpreter as the fall-back.  The variable is read on every call. */
 int32_t dbx_eval_jit_selftest(char* msg, int32_t msg_cap);
 /* Stream of a handle as a cudaStream_t value (for external event timing). */
 int32_t dbx_op_stream(dbx_op* op, void** stream);

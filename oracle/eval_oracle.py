@@ -68,9 +68,36 @@ def int_range(t):
     return (-(1 << (b - 1)), (1 << (b - 1)) - 1) if is_signed(t) else (0, (1 << b) - 1)
 
 
+def int_to_f32(v):
+    """Rust `v as f32` for an integer: rounded ONCE to nearest, ties to even (through f64 a 64-bit
+    integer would round twice: 2^60 + 2^36 + 1 -> 2^60 instead of 2^60 + 2^37)."""
+    a = abs(v)
+    if a < 1 << 24:
+        return float(v)
+    sh = a.bit_length() - 24
+    q, r = a >> sh, a & ((1 << sh) - 1)
+    half = 1 << (sh - 1)
+    if r > half or (r == half and q & 1):
+        q += 1
+    return math.copysign(float(q << sh), v)
+
+
+def round_half_away(x):
+    """f64::round: half away from zero, exactly (floor(|x| + 0.5) is wrong where |x| + 0.5 rounds,
+    e.g. 0.49999999999999994 and odd integers in [2^52, 2^53))."""
+    if math.isnan(x) or math.isinf(x):
+        return x
+    t = math.trunc(x)
+    if abs(x - t) >= 0.5:  # exact: x and trunc(x) are doubles within 1 of each other
+        t += 1 if x > 0 else -1
+    return math.copysign(float(t), x)
+
+
 def cast_as(v, frm, to):
     """Rust `v as to`."""
     if is_float(to):
+        if not is_float(frm):
+            return int_to_f32(int(v)) if to == "F32" else float(int(v))
         x = float(v)
         return float(np.float32(x)) if to == "F32" else x
     if is_float(frm):
@@ -165,9 +192,7 @@ def eval_row(e, row, col_types, r):
         if frm == "BOOL":
             return (cast_as(int(v), "U8", to), True)
         if is_float(frm) and not is_float(to):
-            x = float(v)
-            rounded = math.copysign(math.floor(abs(x) + 0.5), x) if not (math.isnan(x) or math.isinf(x)) else x  # f64::round: half away from zero
-            out = checked_cast(rounded, "F64", to)
+            out = checked_cast(round_half_away(float(v)), "F64", to)
         else:
             out = checked_cast(v, frm, to)
         if out is None:

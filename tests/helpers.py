@@ -1,4 +1,7 @@
 """Shared helpers for the parity tests: compare a GPU result block with the oracle's."""
+import math
+import struct
+
 import numpy as np
 
 from databend_b200 import abi
@@ -79,3 +82,33 @@ def derive_join_rows(kind: str, probe_key, build_key, pairs):
     if kind == "anti":
         return [(int(p), None) for p in np.nonzero(~matched)[0]]
     raise ValueError(kind)
+
+
+INT_TYPES = ["I8", "I16", "I32", "I64", "U8", "U16", "U32", "U64"]
+
+
+def int_type_range(t: str):
+    bits = int(t[1:])
+    return (-(1 << (bits - 1)), (1 << (bits - 1)) - 1) if t[0] == "I" else (0, (1 << bits) - 1)
+
+
+def float_int_boundaries(t: str, ftype: str):
+    """Values of float type `ftype` ("F32" / "F64") where a rounding float -> integer cast to `t` can go
+    wrong: MIN - 1, MIN - 0.5, MIN, MAX, MAX + 0.5, MAX + 1 (each to the nearest value of `ftype`) and
+    both of their neighbours (so MIN - 0.49999999999999994, nextafter(2^63, 0), nextafter(-2^63, -inf),
+    nextafter(2^64, 0) and the like), 2^63 and 2^64, odd integers in [2^52, 2^53), +-0, +-0.5, the
+    subnormals, +-inf and NaN.  Sorted, duplicates removed, as Python floats."""
+    from fractions import Fraction
+    ft = np.float32 if ftype == "F32" else np.float64
+    lo, hi = int_type_range(t)
+    anchors = [Fraction(lo) - 1, Fraction(lo) - Fraction(1, 2), Fraction(lo), Fraction(hi), Fraction(hi) + Fraction(1, 2),
+               Fraction(hi) + 1, Fraction(2) ** 63, -Fraction(2) ** 63, Fraction(2) ** 64, Fraction(1, 2), -Fraction(1, 2)]
+    vals = []
+    with np.errstate(over="ignore"):
+        for a in anchors:
+            x = ft(float(a))  # only needs to land next to the anchor
+            vals += [np.nextafter(x, ft(-np.inf)), x, np.nextafter(x, ft(np.inf))]
+    tiny = np.finfo(ft).smallest_subnormal
+    vals += [0.0, -0.0, tiny, -tiny, np.finfo(ft).tiny, np.inf, -np.inf, 2.0 ** 52 + 1, 2.0 ** 52 + 3, -(2.0 ** 52 + 1), 1.5, -1.5, 2.5, -2.5]
+    by_bits = {struct.pack("<d", float(ft(v))): float(ft(v)) for v in vals}  # keeps -0.0 apart from 0.0
+    return sorted(by_bits.values(), key=lambda v: (v, math.copysign(1.0, v))) + [float("nan")]

@@ -29,9 +29,10 @@ def oracle():
 @pytest.fixture(params=["jit", "interp"])
 def eval_mode(request, monkeypatch):
     """Both builds of the evaluator: a straight-line kernel generated and compiled per expression
-    (default), and the precompiled interpreter (DBX_EVAL_JIT=0)."""
-    if request.param == "interp":
-        monkeypatch.setenv("DBX_EVAL_JIT", "0")
+    (the default; run strict, DBX_EVAL_JIT=2, so that a kernel which fails to compile or launch fails
+    the test instead of falling back to the interpreter), and the precompiled interpreter
+    (DBX_EVAL_JIT=0)."""
+    monkeypatch.setenv("DBX_EVAL_JIT", "2" if request.param == "jit" else "0")
     return request.param
 
 
@@ -161,7 +162,8 @@ def check_against_oracle(cols, rows, e, what=None):
 def test_binary_arithmetic_all_type_pairs(gpu, fn, eval_mode):
     """Every (left type, right type) pair of the ten numeric types, edge values and NULLs included;
     rows whose divisor is zero are exercised separately so that the value comparison runs too.
-    (The generated-kernel build compiles one kernel per pair: it takes a third of the left types.)"""
+    (The generated-kernel build compiles one kernel per pair: it takes a third of the left types
+    here; test_eval_matrix_gpu.py runs it on every pair.)"""
     rng = np.random.default_rng(sum(map(ord, fn)))
     rows = 257
     outcomes = set()

@@ -156,3 +156,100 @@ def test_expression_builder_flattens_to_postfix():
         sx.flatten(big)
     with pytest.raises(DbxError, match="not built"):
         sx.call("sqrt", sx.col(0))
+
+
+# ---- the oracle's numeric conversions against exact rational arithmetic (fractions.Fraction)
+
+INT_TYPES = ["I8", "I16", "I32", "I64", "U8", "U16", "U32", "U64"]
+# 64-bit integers whose correctly rounded f32 differs from the f32 of their f64 (double rounding)
+F32_WITNESSES = {1152921573326323713: 2.0 ** 60 + 2.0 ** 37, -1152921573326323713: -(2.0 ** 60 + 2.0 ** 37),
+                 4611686293305294849: 2.0 ** 62 + 2.0 ** 39, 9223372586610589697: 2.0 ** 63 + 2.0 ** 40}
+
+
+def nearest_even(v, ftype):
+    """`v` (int or Fraction) rounded to the nearest value of ftype, ties to the even significand: the
+    candidates around a first guess are compared by exact distance."""
+    import numpy as np
+    from fractions import Fraction
+    ft, ut = (np.float32, np.uint32) if ftype == "F32" else (np.float64, np.uint64)
+    c = [ft(float(v))]
+    for _ in range(2):
+        c = [np.nextafter(c[0], ft(-np.inf))] + c + [np.nextafter(c[-1], ft(np.inf))]
+    dist = [abs(Fraction(float(x)) - Fraction(v)) for x in c]
+    best = [x for x, d in zip(c, dist) if d == min(dist)]
+    if len(best) == 2:
+        best = [x for x in best if not int(np.asarray(x, ft).view(ut)) & 1]
+    assert len(best) == 1
+    return float(best[0])
+
+
+def round_half_away_exact(x):
+    from fractions import Fraction
+    q = Fraction(x)
+    r = math.floor(abs(q) + Fraction(1, 2))
+    return r if q >= 0 else -r
+
+
+def int_range(t):
+    b = int(t[1:])
+    return (-(1 << (b - 1)), (1 << (b - 1)) - 1) if t[0] == "I" else (0, (1 << b) - 1)
+
+
+def conversion_inputs(t):
+    """Type boundaries, the double-rounding witnesses, seeded uniform values and seeded values at and
+    next to the f32 / f64 rounding ties, all inside the range of `t`."""
+    import random
+    lo, hi = int_range(t)
+    rng = random.Random(t)
+    vals = {lo, lo + 1, hi - 1, hi, 0, 1, (1 << 24) + 1, (1 << 53) + 1, -(1 << 24) - 1, -(1 << 53) - 1}
+    vals.update(F32_WITNESSES)
+    vals.update(rng.randint(lo, hi) for _ in range(1000))
+    bits = int(t[1:])
+    for p in (p for p in (24, 53) if p < bits):
+        for _ in range(300):
+            n = rng.randint(p + 1, bits)
+            m = rng.randrange(1 << (n - 1), 1 << n) | 1 << (n - p - 1)  # n significant bits, bit n-p-1 set ...
+            m &= ~((1 << (n - p - 1)) - 1)                                # ... and nothing below it: a tie
+            for d in (-1, 0, 1):
+                vals.update((m + d, -(m + d)))
+    return sorted(v for v in vals if lo <= v <= hi)
+
+
+@pytest.mark.parametrize("t", INT_TYPES)
+def test_integer_to_float_conversions_round_once_to_nearest_even(t):
+    """Rust `x as f32` / `x as f64` for every integer type, through cast_as, checked_cast and a
+    CAST / TRY_CAST over a column: one rounding, to nearest, ties to even."""
+    vals = conversion_inputs(t)
+    for to in ("F32", "F64"):
+        exp = [nearest_even(v, to) for v in vals]
+        assert [eo.cast_as(v, t, to) for v in vals] == exp, (t, to)
+        assert [eo.checked_cast(v, t, to) for v in vals] == exp, (t, to)
+        for try_cast in (0, 1):
+            rt, nullable, got, oks = eo.evaluate(("cast", ("col", 0), to, try_cast), [(t, vals, None)])
+            assert rt == to and all(oks) and got == exp, (t, to, try_cast)
+    for v, f in F32_WITNESSES.items():
+        if int_range(t)[0] <= v <= int_range(t)[1]:
+            assert eo.cast_as(v, t, "F32") == f == nearest_even(v, "F32"), (t, v)
+
+
+@pytest.mark.parametrize("ftype", ["F32", "F64"])
+@pytest.mark.parametrize("t", INT_TYPES)
+def test_float_to_integer_cast_rounds_half_away_and_accepts_exactly_min_to_max(t, ftype):
+    """CAST / TRY_CAST of a float to an integer rounds half away from zero, then is checked: at every
+    boundary value the cast succeeds exactly when the exactly rounded value lies in [MIN, MAX]."""
+    from helpers import float_int_boundaries
+    lo, hi = int_range(t)
+    xs = float_int_boundaries(t, ftype)
+    exp = [None if (math.isnan(x) or math.isinf(x)) else round_half_away_exact(x) for x in xs]
+    exp = [r if (r is not None and lo <= r <= hi) else None for r in exp]
+    assert any(r is None for r in exp) and any(r is not None for r in exp)
+    for x, r in zip(xs, exp):
+        assert eo.checked_cast(eo.round_half_away(x), "F64", t) == r, (t, ftype, x)
+    rt, nullable, got, oks = eo.evaluate(("cast", ("col", 0), t, 1), [(ftype, xs, None)])
+    assert rt == t and nullable
+    assert oks == [r is not None for r in exp], (t, ftype)
+    assert [g for g, ok in zip(got, oks) if ok] == [r for r in exp if r is not None], (t, ftype)
+    first_bad = next(i for i, r in enumerate(exp) if r is None)
+    with pytest.raises(eo.EvalFailure, match="number overflowed") as ei:
+        eo.evaluate(("cast", ("col", 0), t, 0), [(ftype, xs, None)])
+    assert ei.value.row == first_bad
